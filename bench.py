@@ -3,6 +3,14 @@
 
     python bench.py --gpus N --steps K --warmup W            # the CUDA product (default N=1)
     python bench.py --impl reference --steps K --warmup W     # the reference's CPU/OpenMP path
+    python bench.py ... --dump-outputs DIR                    # also write what the last timed step computed
+
+--dump-outputs DIR writes, after the timed regions of the headline workload (rank 0's slab when N > 1), what a caller
+of the timed path receives from its last step, one DIR/<name>.npy each: accepted_dt (float64, the computeStep return
+values of the timed steps), matric_potential_maps (float32 [layers, rows, cols], the maps the e2e region downloads),
+total_potential and water_content (float64 per node; temperature too with --heat).  An array larger than its cap is
+replaced by the same seeded sample of its flattened values on every run: 56 MiB + 8 B per timed step at most.  The inputs are a
+deterministic function of the arguments, so two builds run with the same arguments can be compared file by file.
 
 A "step" is one computeStep() (soilFluxes3D.cpp:1785) = one accepted water time step of the
 catchment: Picard approximations, each an assembly pass and a batch of Jacobi sweeps.  The
@@ -48,6 +56,8 @@ RAIN_MM_H = 40.0                                                # peak hour of t
 # generator, forcing and warm-up): 7.5 GB of reference state, ~2-3 s per computeStep on 16 cores; the timed part is
 # bounded by a wall-time budget, the number of steps actually timed is reported.
 C4_SLAB = dict(rows=512, cols=4096, soil_layers=20)            # per-GPU slab of BASELINE.json configs[3] (8 of them = 4096 x 4096)
+DUMP_MAP_VALUES = 11 * 1024 * 1024                              # float32 map values kept by --dump-outputs: all 11 maps of C2 (44 MiB)
+DUMP_NODE_VALUES = 1 << 19                                      # float64 node values kept per field (4 MiB)
 
 
 def measured_peak():
@@ -157,6 +167,27 @@ def cpu_run(sample: dict, steps: int, warmup: int, budget_s: float):
     }
 
 
+def _seeded_sample(a: np.ndarray, cap: int, seed: int = 0) -> np.ndarray:
+    """`a` itself when it has at most `cap` values, else `cap` of its flattened values at positions fixed by `seed`"""
+    if a.size <= cap:
+        return np.array(a)
+    idx = np.sort(np.random.default_rng(seed).choice(a.size, cap, replace=False))
+    return np.ascontiguousarray(a).reshape(-1)[idx]
+
+
+def last_step_outputs(sf, N, dts, maps, heat) -> dict:
+    """what a caller of the timed path holds after its last step (see --dump-outputs in the module docstring)"""
+    from criteria3d_b200 import Field
+    out = {"accepted_dt": np.asarray(dts, dtype=np.float64),
+           "matric_potential_maps": _seeded_sample(maps, DUMP_MAP_VALUES)}
+    fields = [("total_potential", Field.TOTAL_POTENTIAL), ("water_content", Field.WATER_CONTENT)]
+    if heat:
+        fields.append(("temperature", Field.TEMPERATURE))
+    for name, f in fields:
+        out[name] = _seeded_sample(sf.get_field(f, 0, N), DUMP_NODE_VALUES)
+    return out
+
+
 def config_name(args, world) -> str:
     """BASELINE.json configuration the shape corresponds to (C2 is the headline single-GPU workload)"""
     shape = (args.rows * world, args.cols, args.soil_layers)
@@ -206,10 +237,12 @@ def timed_region(sf, steps, stream, barrier, *, e2e=None):
     return ev0.elapsed_time(ev1), wall, float(sum(dts)), dts, [1e3 * t / max(steps, 1) for t in tcall]
 
 
-def run_workload(sf, args, shape, rank, local_rank, world, steps, warmup, *, heat=False, saturated_bottom=False, with_e2e=True):
+def run_workload(sf, args, shape, rank, local_rank, world, steps, warmup, *, heat=False, saturated_bottom=False, with_e2e=True,
+                 keep_outputs=False):
     """Set up `shape` = (rows per GPU, cols, soil layers) on this rank (a row slab when world > 1), warm up, then time
     the SAME `steps` accepted steps twice from the same saved state: device-resident (value) and end to end through
-    the C ABI with host buffers (e2e).  Returns this rank's measurements (times already max-reduced over ranks)."""
+    the C ABI with host buffers (e2e).  Returns this rank's measurements (times already max-reduced over ranks) and,
+    with keep_outputs (needs with_e2e), what the last timed step computed under "outputs"."""
     import torch
     import torch.distributed as dist
     from criteria3d_b200 import Field
@@ -295,6 +328,10 @@ def run_workload(sf, args, shape, rank, local_rank, world, steps, warmup, *, hea
         res["profiled_same_steps"] = bool(dts_p == dts and (cp1["sweeps"] - cp0["sweeps"]) == res["sweeps"])
     res["ktimes"], res["ms_profiled"] = ktimes, ms_prof
     res["clocks"] = clocks.stop()
+    if keep_outputs:
+        assert with_e2e and steps > 0, "the outputs of the last timed step are those of the e2e region"
+        # the e2e region runs last among the timed ones (region 3 replays the same steps to the same state)
+        res["outputs"] = last_step_outputs(sf, N, dts_e, out_np[(steps - 1) & 1], heat)
 
     # max over ranks of the device times; owned nodes summed (every rank executes the same sweeps on its slab)
     if world > 1:
@@ -321,10 +358,18 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="skip the C4-slab block (512 x 4096 x (1+20) per GPU)")
     ap.add_argument("--no-parity-check", action="store_true", help="skip the N-rank slab-vs-reference parity check")
-    ap.add_argument("--c4-steps", type=int, default=20)
+    ap.add_argument("--c4-steps", type=int, default=None, help="timed steps of the C4-slab block (default: --steps)")
     ap.add_argument("--saturated-bottom", action="store_true", help="config 4: lower third of the layers start saturated")
     ap.add_argument("--heat", action="store_true", help="config 3: coupled heat transport (not the headline workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.c4_steps is None:
+        args.c4_steps = args.steps
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA product (--impl b200)")
+    if args.dump_outputs is not None and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step (--steps >= 1)")
     warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -378,7 +423,11 @@ def main():
 
     # weak scaling: every GPU owns a rows x cols slab of a (world * rows) x cols catchment
     r = run_workload(sf, args, (args.rows, args.cols, args.soil_layers), rank, local_rank, world, args.steps, warmup,
-                     heat=args.heat, saturated_bottom=args.saturated_bottom)
+                     heat=args.heat, saturated_bottom=args.saturated_bottom, keep_outputs=args.dump_outputs is not None and rank == 0)
+    if "outputs" in r:
+        args.dump_outputs.mkdir(parents=True, exist_ok=True)
+        for name, a in r.pop("outputs").items():
+            np.save(args.dump_outputs / f"{name}.npy", a)
     c4 = None
     headline_c2 = (args.rows, args.cols, args.soil_layers) == (WORKLOAD["rows"], WORKLOAD["cols"], WORKLOAD["soil_layers"]) and not args.heat
     if headline_c2 and not args.no_c4:

@@ -24,7 +24,7 @@ def test_header_and_binding_agree():
 def test_library_exports_every_declared_symbol(lib):
     if not lib.exists():
         if lib == REFERENCE_LIB:
-            pytest.skip("oracle/_ref not built here (needs /root/reference)")
+            pytest.skip("oracle/_ref not built (make -C oracle ref REF=<CRITERIA3D checkout>)")
         pytest.fail(f"{lib} missing: run __graft_entry__.build()")
     h = ctypes.CDLL(str(lib), mode=ctypes.RTLD_LOCAL)
     missing = [s for s in DECLARED if not hasattr(h, s)]

@@ -43,7 +43,7 @@ def test_one_object_links_against_reference_and_product(tmp_path):
     exes = _build(tmp_path)
     assert "product" in exes, "libsf3d_b200.so missing: build the product first"
     if "reference" not in exes:
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+        pytest.skip("oracle/_ref not built (make -C oracle ref REF=<CRITERIA3D checkout>)")
     tokens = _run(exes["reference"])
     assert tokens[0] == "steps" and int(tokens[1]) > 0
     assert tokens[-2:] == ["index_error", "-1111.0"]
@@ -53,7 +53,7 @@ def test_one_object_links_against_reference_and_product(tmp_path):
 def test_swapping_the_library_keeps_the_numbers(tmp_path):
     exes = _build(tmp_path)
     if "reference" not in exes:
-        pytest.skip("oracle/_ref not shipped with this snapshot")
+        pytest.skip("oracle/_ref not built (make -C oracle ref REF=<CRITERIA3D checkout>)")
     ref, prod = _run(exes["reference"]), _run(exes["product"])
     assert len(ref) == len(prod)
     for a, b in zip(prod, ref):

@@ -62,7 +62,7 @@ def _cases():
             "all nodata": (np.full((4, 5), -9999, np.float32), 3.0)}
 
 
-@pytest.mark.skipif(not GIS_REF.exists(), reason="oracle/_ref/libgis_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not GIS_REF.exists(), reason="oracle/_ref/libgis_ref.so not built (make -C oracle ref REF=<CRITERIA3D checkout>)")
 @pytest.mark.parametrize("name", sorted(_cases()))
 def test_slope_aspect_boundary_match_reference_library(name):
     import sys
@@ -101,7 +101,7 @@ def _ref_read(noext, cap=4_000_000):
     return v[: r.value * c.value].reshape(r.value, c.value).copy(), (cell.value, xll.value, yll.value, flag.value)
 
 
-@pytest.mark.skipif(not GIS_REF.exists(), reason="oracle/_ref/libgis_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not GIS_REF.exists(), reason="oracle/_ref/libgis_ref.so not built (make -C oracle ref REF=<CRITERIA3D checkout>)")
 def test_flt_files_interchange_with_the_reference_reader_and_writer(tmp_path):
     import ctypes as C
     vals = np.arange(35, dtype=np.float32).reshape(5, 7) * 1.25
