@@ -44,14 +44,11 @@ int  comm_world();
 int  comm_rank();
 void comm_clear_halo();
 void comm_add_halo_peer(int peer, uint32_t nSend, const uint32_t *sendIdx, uint32_t nRecv, const uint32_t *recvIdx);
-void comm_allreduce(double *devValues, int count, bool isMax, Ctrl *ctrl);
 void comm_mailbox_export(unsigned char out[64]);
 void comm_mailbox_import(int peer, const unsigned char handle[64]);
-void comm_halo(double *x, const Ctrl *ctrl);
-void comm_mark_boundary(uint16_t *pid);     // boundary rows of the fused multi-GPU sweep (after every pattern build)
+void comm_mark_boundary(uint16_t *pid);     // boundary rows of the peer-transport sweep (after every pattern build)
 void comm_ipc_export(double *x0, double *x1, unsigned char out[128]);
 void comm_ipc_import(int peer, const unsigned char handles[128], uint32_t n, const uint32_t *remoteIdx);
-bool comm_direct_halo();
 
 // ---- kernels -----------------------------------------------------------------------------
 int  reduce_blocks(uint32_t n);          // grid size used by all reducing kernels for n rows
@@ -85,7 +82,6 @@ void k_heat_jacobi(const SF3DView &v, const double *xin, double *xout, int maxIt
 void k_heat_post(const SF3DView &v, const double *x, double dtHeat, double dtWater, int mode);
 void k_heat_accept(const SF3DView &v, double dtHeat, double dtWater);
 void k_heat_copy_T(const SF3DView &v, int mode);
-void k_halo(double *x);
 void read_ctrl(const SF3DView &v, Ctrl *out);     // async copy to pinned + stream sync
 void write_ctrl(const SF3DView &v, const Ctrl *in);
 

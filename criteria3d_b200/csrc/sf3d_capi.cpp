@@ -125,7 +125,7 @@ void fill_view()
     v.lidx = S.lidx.d; v.larea = S.larea.d; v.lflow = S.lflow.d; v.lgeom = S.lgeom;
     v.H = S.H.d; v.oldH = S.oldH.d; v.bestH = S.bestH; v.Se = S.Se.d; v.SeOld = S.SeOld; v.K = S.K.d;
     v.wFlow = S.wFlow; v.sink = S.sink.d; v.pond = S.pond.d;
-    v.mcol = S.mcol; v.pid = S.patternsOk ? S.pid : nullptr; v.pattern = S.patternsOk ? S.pattern : nullptr; v.mval = S.mval;
+    v.mcol = S.mcol; v.pid = S.pid; v.pattern = S.patternsOk ? S.pattern : nullptr; v.mval = S.mval;
     v.hotPid = S.hotPid; memcpy(v.hotOff, S.hotOff, sizeof v.hotOff); v.b = S.b; v.cap = S.cap; v.x0 = S.x0; v.x1 = S.x1;
     v.soil = S.dSoil; v.rough = S.dRough;
     v.culverts = S.culverts.empty() ? nullptr : S.dCulv;
@@ -207,7 +207,7 @@ uint8_t sync_to_device(bool finalizeTopology = true)
         k_link_geometry(S.eng.v, &ok);
         if (S.heat) k_heat_geometry(S.eng.v);
         S.patternsOk = k_build_patterns(S.eng.v, S.pid, S.pattern, &S.hotPid, S.hotOff) && getenv("SF3D_EXPLICIT_INDEX") == nullptr;
-        if (S.patternsOk) comm_mark_boundary(S.pid);
+        comm_mark_boundary(S.pid);
         fill_view();
         S.topoDirty = false;
         if (!ok)

@@ -414,7 +414,7 @@ SF3D_HD void sf3d_row_store(const SF3DView &v, uint32_t i, double dt, const doub
 // all), other rows read their ten offsets from the small pattern table; without: the explicit array.
 SF3D_HD void sf3d_row_cols(const SF3DView &v, uint32_t i, uint32_t *j)
 {
-    if (v.pid)
+    if (v.pattern)
     {
         const uint32_t p = v.pid[i] & SF3D_PID_MASK;
         if (p == v.hotPid)
@@ -440,7 +440,7 @@ SF3D_HD void sf3d_row_cols(const SF3DView &v, uint32_t i, uint32_t *j)
 // and the assembly kernel is bound by fp64 issue, not by these L1-resident loads)
 SF3D_HD const int32_t *sf3d_row_pattern(const SF3DView &v, uint32_t i)
 {
-    return v.pid ? v.pattern + (size_t)(v.pid[i] & SF3D_PID_MASK) * SF3D_NLINK : nullptr;
+    return v.pattern ? v.pattern + (size_t)(v.pid[i] & SF3D_PID_MASK) * SF3D_NLINK : nullptr;
 }
 SF3D_HD uint32_t sf3d_col_index(const SF3DView &v, const int32_t *__restrict__ off, uint32_t i, int c)
 {

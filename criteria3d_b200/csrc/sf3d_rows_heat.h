@@ -830,7 +830,7 @@ SF3D_HD double sf3d_row_heat_jacobi(const SF3DView &v, uint32_t i, const double 
     if (xnewOut) *xnewOut = xold;
     if (i < v.Ns || SF3D_LDS(v.hdiag + i) == 0.) { xout[i] = xold; return 0.; }
     uint32_t j[SF3D_NLINK];
-    if (v.pid) sf3d_row_cols(v, i, j);          // j[c]: COLUMN order (Up, Lateral 0..7, Down)
+    if (v.pattern) sf3d_row_cols(v, i, j);      // j[c]: COLUMN order (Up, Lateral 0..7, Down)
     else
     {
         const uint32_t m = v.meta[i];

@@ -139,7 +139,9 @@ struct SF3DView {
     // linear system, COLUMN-major: [col*N + i]; mcol is static
     uint32_t *mcol;
     // pattern-compressed column indices: mcol[c][i] == i + pattern[pid[i]*10 + c] for every node
-    // (verified bit-exactly at finalize); null when the graph has too many distinct link patterns
+    // (verified bit-exactly at finalize).  pattern is null when the graph has too many distinct link patterns
+    // (or SF3D_EXPLICIT_INDEX is set); pid is set in either case, since it also carries the row class (see
+    // SF3D_PID_SKIP).  Both null only in single-rank views without a pattern build.
     const uint16_t *pid;
     const int32_t *pattern;
     uint32_t hotPid;                // the most frequent pattern (interior nodes) and its offsets, held in

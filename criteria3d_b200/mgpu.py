@@ -58,8 +58,7 @@ def setup_slab(sf: SoilFluxes3D, rows: int, cols: int, n_soil_layers: int, rank:
 def wire_direct_halo(sf: SoilFluxes3D, slab: Slab, peers) -> None:
     """Exchange the CUDA IPC handles of every rank's solution buffers and mailbox and tell the library where each
     send entry lives in the neighbour's numbering (= the neighbour's recv list towards this rank)."""
-    reduce_direct = os.environ.get("SF3D_DIRECT_REDUCE", "1") != "0"
-    blob = sf.ipc_export() + (sf.mailbox_export() if reduce_direct else bytes(64))
+    blob = sf.ipc_export() + sf.mailbox_export()
     blobs = [None] * slab.world
     dist.all_gather_object(blobs, blob)
     for p in peers:
@@ -67,7 +66,6 @@ def wire_direct_halo(sf: SoilFluxes3D, slab: Slab, peers) -> None:
         o_peers, _o_send, o_recv = other.halo()
         remote = o_recv[o_peers.index(slab.rank)]
         _ok(sf.ipc_import(p, blobs[p][:128], remote), "sf3d_ext_ipc_import")
-    if reduce_direct:
-        for p in range(slab.world):
-            if p != slab.rank:
-                _ok(sf.mailbox_import(p, blobs[p][128:192]), "sf3d_ext_mailbox_import")
+    for p in range(slab.world):
+        if p != slab.rank:
+            _ok(sf.mailbox_import(p, blobs[p][128:192]), "sf3d_ext_mailbox_import")

@@ -344,17 +344,16 @@ uint8_t sf3d_ext_set_halo(uint32_t n_peers, const int32_t *peers,
                           const uint32_t *recv_count, const uint32_t *recv_idx,
                           uint64_t n_global_nodes);
 
-/* product only, optional after sf3d_ext_set_halo: direct halo.  Each rank exports CUDA IPC handles of
- * its two solution buffers (128 bytes); a rank that imports its neighbours' handles, together with the
- * position of each of its send entries in the neighbour's numbering (the neighbour's recv list),
- * stores its boundary values straight into the neighbours' ghost rows through NVLink peer memory
- * from a kernel that follows the sweep, instead of pack -> ncclSend/ncclRecv -> unpack. */
+/* product only, optional after sf3d_ext_set_halo: the peer-memory transport.  Each rank exports CUDA IPC
+ * handles of its two solution buffers (128 bytes) and of a small mailbox (64 bytes); it imports the buffer
+ * handles of every neighbour, together with the position of each of its send entries in the neighbour's
+ * numbering (the neighbour's recv list), and the mailboxes of ALL other ranks.  With all of them imported
+ * (at most 4 neighbours; sf3d_ext_ipc_import fails beyond that) every sweep is one kernel that stores the
+ * boundary rows straight into the neighbours' ghost rows over NVLink, and the residual / Courant / balance
+ * all-reduces run inside the producing kernels through the mailboxes (deterministic rank-order fold);
+ * otherwise the library uses NCCL.  Wire all ranks or none: the choice must be the same on every rank. */
 uint8_t sf3d_ext_ipc_export(uint8_t handles[128]);
 uint8_t sf3d_ext_ipc_import(int peer, const uint8_t handles[128], uint32_t n, const uint32_t *remote_idx);
-/* product only, optional: direct reductions.  Every rank exports the CUDA IPC handle of a small mailbox
- * and imports the mailboxes of ALL other ranks; the residual / Courant / balance all-reduces then run as
- * one warp-sized kernel that stores into the peers' mailboxes over NVLink (deterministic rank-order fold)
- * instead of ncclAllReduce. */
 uint8_t sf3d_ext_mailbox_export(uint8_t handle[64]);
 uint8_t sf3d_ext_mailbox_import(int peer, const uint8_t handle[64]);
 

@@ -34,6 +34,7 @@ def slab_parity(gpu, rank: int, world: int, *, heat: bool = False, nccl: bool = 
     # save_all: heat flux save mode All (every flux type kept per link), which also runs the water-flux snapshot pass
     hf_mode = 2 if (heat and save_all) else None
     slab, lc = setup_slab(gpu, R, C, L, rank, world, heat=heat, require_direct=not nccl, heat_flux_mode=hf_mode, **cat_kw)
+    launches0 = gpu.counters()["kernel_launches"]
 
     def run(sf, cat):
         dts = []
@@ -43,13 +44,14 @@ def slab_parity(gpu, rank: int, world: int, *, heat: bool = False, nccl: bool = 
             dts += run_hours(sf, cat, [mm], max_steps=max_steps)
         return dts
     dts = run(gpu, lc)
+    launches = int(gpu.counters()["kernel_launches"] - launches0)
     chk = SoilFluxes3D(checker_path())
     cat = Catchment(R, C, L, heat=heat, **cat_kw)
     setup(chk, cat, threads=threads, heat_flux_mode=hf_mode)
     dts_ref = run(chk, cat)
 
     out = {"world": world, "grid": f"{R}x{C}x(1+{L})" + (" coupled heat" if heat else "") + (", save mode All" if hf_mode else "") + (" saturated lower third (C4 recipe)" if c4 else ""), "checker": chk.backend,
-           "halo": getattr(gpu, "halo_mode", "?"), "steps": len(dts), "dt_sequence_equal": dts == dts_ref, "ok": True, "why": []}
+           "halo": getattr(gpu, "halo_mode", "?"), "steps": len(dts), "dt_sequence_equal": dts == dts_ref, "launches": launches, "ok": True, "why": []}
     if dts != dts_ref:
         out["ok"] = False
         out["why"].append("accepted time steps differ")
@@ -101,7 +103,8 @@ def slab_parity(gpu, rank: int, world: int, *, heat: bool = False, nccl: bool = 
 
 
 def reduce_over_ranks(out: dict) -> dict:
-    """worst case over the ranks (every rank checked its own slab)"""
+    """worst case over the ranks (every rank checked its own slab).  Every rank must have launched the same kernels:
+    the ranks take the same decisions (same transport, same sweeps), so unequal counts mean a mixed-form run."""
     import torch.distributed as dist
     alls = [None] * dist.get_world_size()
     dist.all_gather_object(alls, out)
@@ -109,6 +112,10 @@ def reduce_over_ranks(out: dict) -> dict:
     merged["ok"] = all(o["ok"] for o in alls)
     merged["dt_sequence_equal"] = all(o["dt_sequence_equal"] for o in alls)
     merged["why"] = sorted({w for o in alls for w in o["why"]})
+    launches = [o["launches"] for o in alls]
+    if len(set(launches)) != 1:
+        merged["ok"] = False
+        merged["why"].append(f"kernel launches differ between ranks: {launches}")
     for k in ("max_dH_rel", "max_dtheta", "max_dSe", "max_dT_rel", "total_water_rel"):
         if k in merged:
             merged[k] = max(o[k] for o in alls)

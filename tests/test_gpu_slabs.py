@@ -4,6 +4,7 @@ process group, CUDA-IPC peer memory of the same device, no NCCL), so the multi-r
 the mailbox all-reduce and its time-out are exercised on a one-GPU box too; the host-side partition logic is
 covered on CPU with gloo (tests/test_partition.py)."""
 import os
+import re
 import subprocess
 import sys
 from pathlib import Path
@@ -25,14 +26,39 @@ def _torchrun(world, port, *args, env_extra=None, timeout=900):
     return subprocess.run(cmd, capture_output=True, text=True, timeout=timeout, env=env)
 
 
-@pytest.mark.parametrize("world,heat", [(2, False), (4, False), (8, False), (2, True), (4, True), (4, "c4"), (2, "heat-all")])
+def _result_line(stdout):
+    return next(ln for ln in stdout.splitlines() if ln.startswith("[mgpu_slab_check]"))
+
+
+def _launches(line):
+    return int(re.search(r"'launches': (\d+)", line).group(1))
+
+
+@pytest.mark.parametrize("world,heat", [(2, False), (4, False), (8, False), (2, True), (4, True), (4, "c4"), (2, "heat-all"),
+                                        (2, "explicit-index"), (2, "nccl")])
 def test_slabs_match_oracle(world, heat):
-    """water storm, coupled heat, and the C4 recipe (20 soil layers, saturated lower third, free drainage) at small size"""
-    args = {"c4": ["--c4"], "heat-all": ["--heat", "--save-all"]}.get(heat, ["--heat"] if heat else [])
-    r = _torchrun(world, 29600 + world + {"c4": 20, "heat-all": 30}.get(heat, 10 if heat else 0), *args)
+    """water storm, coupled heat, and the C4 recipe (20 soil layers, saturated lower third, free drainage) at small size.
+    explicit-index: the water storm without pattern compression, which must take the same peer-memory sweep (same
+    launches as with patterns).  nccl: the water storm on the NCCL fallback (two devices: NCCL cannot put two ranks
+    on one GPU)."""
+    import torch
+    if heat == "nccl" and torch.cuda.device_count() < 2:
+        pytest.skip("the NCCL transport needs two devices")
+    args = {"c4": ["--c4"], "heat-all": ["--heat", "--save-all"]}.get(heat, ["--heat"] if heat is True else [])
+    env = {"explicit-index": {"SF3D_EXPLICIT_INDEX": "1"}, "nccl": {"SF3D_DIRECT_HALO": "0"}}.get(heat)
+    port = 29600 + world + {"c4": 20, "heat-all": 30, "explicit-index": 40, "nccl": 50}.get(heat, 10 if heat else 0)
+    r = _torchrun(world, port, *args, env_extra=env)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
     assert "[mgpu_slab_check] ok" in r.stdout
-    print(r.stdout.strip().splitlines()[-1])
+    line = _result_line(r.stdout)
+    if heat == "nccl":
+        assert "'halo': 'nccl'" in line, line
+    if heat == "explicit-index":
+        assert "'halo': 'peer-memory'" in line, line
+        default = _torchrun(world, port + 1)
+        assert default.returncode == 0, default.stdout[-3000:] + default.stderr[-3000:]
+        assert _launches(line) == _launches(_result_line(default.stdout)), (line, _result_line(default.stdout))
+    print(line)
 
 
 def test_silent_peer_is_an_error_not_a_numerical_event():
