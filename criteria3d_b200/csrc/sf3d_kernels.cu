@@ -29,7 +29,9 @@
 namespace sf3d {
 
 #define SF3D_BLOCK 256
-#define SF3D_MAX_BLOCKS (148 * 8)
+#ifndef SF3D_MAX_BLOCKS
+#define SF3D_MAX_BLOCKS (148 * 8)           // grid cap of the sweep and of every other reducing / streaming kernel
+#endif
 #ifndef SF3D_WIDE_BLOCKS
 #define SF3D_WIDE_BLOCKS (148 * 48)         // grid cap of the fp64-heavy node / assembly kernels (a multiple of every
                                             // residency below, short tail wave)
