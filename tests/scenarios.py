@@ -406,18 +406,43 @@ TOLERANCES = {
 }
 
 
-def compare(a: dict, b: dict, *, exact: bool, h_rel=1e-6, theta_abs=1e-7, flow_rel=1e-6, flow_head_tol=0.0, skip_stale_links=True):
-    """exact: bit-identical (oracle restatement vs reference, same libm).  Otherwise the fp64
-    tolerances stated in tests/test_gpu_parity.py."""
-    assert set(a) == set(b)
-    if exact:
-        for k in a:
-            assert np.array_equal(np.asarray(a[k]), np.asarray(b[k]), equal_nan=True), k
-        return
-    assert np.array_equal(a["dts"], b["dts"]), "accepted time-step sequence"
+def assert_bit_identical(a: dict, b: dict, what: str):
+    """the same quantities, equal bit for bit (NaN equal to NaN)"""
+    assert set(a) == set(b), what
+    for k in a:
+        assert np.array_equal(np.asarray(a[k]), np.asarray(b[k]), equal_nan=True), f"{what}: {k} differs"
+
+
+def assert_lockstep(a: dict, b: dict, psi):
+    """Snapshots after ONE computeStep from the same state: the same accepted dt and approximation count,
+    |dH| <= 1e-9 * max(1, |psi|) with psi the checker's matric potential after the step, and |dtheta| <= 1e-10
+    on the soil nodes."""
+    assert np.array_equal(a["dts"], b["dts"]), "accepted dt"
     assert a["counters"][0] == b["counters"][0], "approximation count"
+    assert np.max(np.abs(a["TOTAL_POTENTIAL"] - b["TOTAL_POTENTIAL"]) / np.maximum(1.0, np.abs(psi))) <= 1e-9
+    ns = int(b["n_surface"])
+    assert np.max(np.abs(a["WATER_CONTENT"][ns:] - b["WATER_CONTENT"][ns:])) <= 1e-10
+
+
+def compare(a: dict, b: dict, *, exact: bool, h_rel=1e-6, theta_abs=1e-7, flow_rel=1e-6, flow_head_tol=0.0,
+            h_abs=None, totals_rel=None, sweeps=False, mbe_abs=None):
+    """exact: bit-identical (oracle restatement vs reference, same libm).  Otherwise the fp64
+    tolerances stated in tests/test_gpu_parity.py.  Off unless given: an absolute head bound h_abs [m], a
+    relative bound totals_rel for the boundary totals other than flow_rel, equal sweep counts, and a bound
+    mbe_abs [m3] on the difference of the last step's mass-balance errors (it scales with the rain)."""
+    if exact:
+        assert_bit_identical(a, b, "exact")
+        return
+    assert set(a) == set(b)
+    first = next((k for k, (x, y) in enumerate(zip(a["dts"], b["dts"])) if x != y), None)
+    assert np.array_equal(a["dts"], b["dts"]), f"accepted time-step sequences differ from step {first}"
+    assert a["counters"][0] == b["counters"][0], "approximation count"
+    if sweeps:
+        assert a["counters"][1] == b["counters"][1], "sweep count"
     H, Hb = a["TOTAL_POTENTIAL"], b["TOTAL_POTENTIAL"]
     assert np.max(np.abs(H - Hb) / np.maximum(1.0, np.abs(Hb))) <= h_rel
+    if h_abs is not None:
+        assert np.max(np.abs(H - Hb)) <= h_abs, "total potential, absolute"
     assert np.max(np.abs(a["WATER_CONTENT"] - b["WATER_CONTENT"])) <= theta_abs
     assert np.max(np.abs(a["DEGREE_OF_SATURATION"] - b["DEGREE_OF_SATURATION"])) <= 1e-6
     K, Kb = a["WATER_CONDUCTIVITY"], b["WATER_CONDUCTIVITY"]
@@ -436,7 +461,9 @@ def compare(a: dict, b: dict, *, exact: bool, h_rel=1e-6, theta_abs=1e-7, flow_r
         assert np.max(np.abs(x - y)) <= flow_rel * scale + 1e-12 + flow_head_tol * float(np.sum(b["dts"])), k
     assert a["total_water"] == np.float64(b["total_water"]) or abs(a["total_water"] - b["total_water"]) <= 1e-9 * abs(b["total_water"])
     bt, btb = a["boundary_totals"], b["boundary_totals"]
-    assert np.all(np.abs(bt - btb) <= flow_rel * np.abs(btb) + 1e-12)
+    assert np.all(np.abs(bt - btb) <= (flow_rel if totals_rel is None else totals_rel) * np.abs(btb) + 1e-12), "boundary totals"
+    if mbe_abs is not None:
+        assert abs(a["mbe_mbr"][0] - b["mbe_mbr"][0]) <= mbe_abs, "mass-balance error of the last step"
     if "TEMPERATURE" in a:
         # heat: the product iterates Jacobi where the reference sweeps Gauss-Seidel (same fixed point,
         # stopping tolerance 1e-10 K on the update); temperatures rel 1e-6, boundary diagnostics rel 1e-5

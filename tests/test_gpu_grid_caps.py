@@ -16,17 +16,18 @@ each other (same grid, same partials, same fold order: tests/test_gpu_persistent
 
 Real caps.  The default product on both sides of the persistent-solve limit (N <= 303 104, DESIGN section 4) and on a
 1.9 M node window past the wide cap, lock-step on the first step and over the first 20 accepted steps of a
-40 mm/h hour; tolerances of tests/test_gpu_parity.py."""
+40 mm/h hour; tolerances of tests/test_gpu_parity.py, with equal sweep counts."""
 import time
 from pathlib import Path
 
 import numpy as np
 import pytest
 
-from criteria3d_b200 import BoundaryType, Field, SoilFluxes3D
+from criteria3d_b200 import Field, SoilFluxes3D
 from criteria3d_b200.synth import Catchment, _ok, setup
 from oracle import ORACLE_LIB
-from scenarios import HEAT_SCENARIOS, SCENARIOS, TOLERANCES, compare, culvert_outlet
+from scenarios import (HEAT_SCENARIOS, SCENARIOS, TOLERANCES, assert_bit_identical, assert_lockstep, compare, culvert_outlet,
+                       snapshot)
 from test_gpu_parity import test_index_maps_bit_exact as _index_maps_bit_exact
 from test_gpu_parity import test_pattern_compressed_indices_are_bit_identical as _pattern_indices_bit_identical
 from test_gpu_persistent_solve import _with_mode
@@ -44,13 +45,6 @@ def smallgrid():
     sf = SoilFluxes3D(SMALLGRID)
     assert sf.backend == "b200"
     return sf
-
-
-def _assert_bit_identical(a, b, what):
-    for key in a:
-        x, y = np.asarray(a[key]), np.asarray(b[key])
-        if x.dtype.kind in "fiu" and x.shape == y.shape:
-            assert np.array_equal(x, y, equal_nan=True), f"{what}: {key} differs between the two solve paths"
 
 
 # ---- small-grid build ---------------------------------------------------------------------------------------------
@@ -73,7 +67,7 @@ def test_small_grid_both_solve_paths(smallgrid, checker, name):
         compare(out[path], ref, exact=False, **TOLERANCES.get(name, {}))
         if "culvert_total" in ref:
             assert abs(out[path]["culvert_total"] - ref["culvert_total"]) <= 1e-6 * abs(ref["culvert_total"])
-    _assert_bit_identical(out["persistent"], out["per sweep"], name)
+    assert_bit_identical(out["persistent"], out["per sweep"], f"{name}, persistent vs per sweep")
     # the persistent solve is one launch per solve, the other path at least four (its first batch)
     assert launches["persistent"] < launches["per sweep"], launches
     approx, sweeps = (int(v) for v in out["persistent"]["counters"])
@@ -95,9 +89,9 @@ RAIN_MM_H = 40.0
 
 
 def _first_steps_of_hour(sf, cat, steps=20):
-    """setup on all host cores, then the first `steps` accepted steps of an hour of RAIN_MM_H.  Returns the state after
-    the first step (lock-step comparison), the state after the last one, the kernel launches and the time spent in
-    computeStep."""
+    """setup on all host cores, then the first `steps` accepted steps of an hour of RAIN_MM_H.  Returns the snapshot
+    after the first step (lock-step comparison) with the matric potential then, the snapshot after the last one, and
+    the kernel launches of and the time spent in computeStep."""
     setup(sf, cat, threads=0)
     sink = np.zeros(cat.n_nodes)
     sink[: cat.n_surface] = cat.rain_sink_source(RAIN_MM_H)
@@ -106,41 +100,15 @@ def _first_steps_of_hour(sf, cat, steps=20):
     t0 = time.perf_counter()
     dts = [sf.computeStep(3600.0)]
     wall = time.perf_counter() - t0
-    first = dict(dt=dts[0], approximations=sf.counters()["approximations"],
-                 H=sf.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes), W=sf.get_field(Field.WATER_CONTENT, 0, cat.n_nodes),
-                 psi=sf.get_field(Field.MATRIC_POTENTIAL, 0, cat.n_nodes))
+    launches = sf.counters()["kernel_launches"] - l0
+    first, psi = snapshot(sf, cat.n_nodes, dts), sf.get_field(Field.MATRIC_POTENTIAL, 0, cat.n_nodes)
+    l0 = sf.counters()["kernel_launches"]
     t0 = time.perf_counter()
     while len(dts) < steps and sum(dts) < 3600.0:
         dts.append(sf.computeStep(3600.0 - sum(dts)))
     wall += time.perf_counter() - t0
-    c = sf.counters()
-    last = dict(dts=np.array(dts), H=sf.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes),
-                W=sf.get_field(Field.WATER_CONTENT, 0, cat.n_nodes),
-                boundary=np.array([sf.getTotalBoundaryWaterFlow(int(b)) for b in
-                                   (BoundaryType.Runoff, BoundaryType.FreeDrainage, BoundaryType.FreeLateralDrainage)]),
-                total_water=np.float64(sf.getTotalWaterContent()),
-                counters=np.array([c["steps"], c["approximations"], c["sweeps"]]), last_mbe=np.float64(c["last_mbe"]))
-    return dict(first=first, last=last, launches=c["kernel_launches"] - l0, wall=wall)
-
-
-def _assert_matches_reference(cat, gpu, ref):
-    f, fr = gpu["first"], ref["first"]
-    # lock-step single step (test_gpu_parity.test_lockstep_single_step)
-    assert f["dt"] == fr["dt"] and f["approximations"] == fr["approximations"], "first step"
-    assert np.max(np.abs(f["H"] - fr["H"]) / np.maximum(1.0, np.abs(fr["psi"]))) <= 1e-9
-    assert np.max(np.abs(f["W"] - fr["W"])[cat.n_surface:]) <= 1e-10
-    # trajectory (test_gpu_parity.test_trajectory)
-    l, lr = gpu["last"], ref["last"]
-    first = next((k for k, (x, y) in enumerate(zip(l["dts"], lr["dts"])) if x != y), None)
-    assert np.array_equal(l["dts"], lr["dts"]), f"accepted time-step sequences differ from step {first}"
-    assert np.array_equal(l["counters"], lr["counters"]), "steps, approximations, sweeps"
-    assert np.max(np.abs(l["H"] - lr["H"]) / np.maximum(1.0, np.abs(lr["H"]))) <= 1e-6
-    assert np.max(np.abs(l["W"] - lr["W"])) <= 1e-7
-    for a, b in zip(l["boundary"], lr["boundary"]):
-        assert a == pytest.approx(b, rel=1e-6, abs=1e-9)
-    assert l["total_water"] == pytest.approx(lr["total_water"], rel=1e-9)
-    sink_total = np.sum(np.abs(cat.rain_sink_source(RAIN_MM_H))) * np.sum(lr["dts"])
-    assert abs(l["last_mbe"] - lr["last_mbe"]) <= 1e-6 * sink_total
+    launches += sf.counters()["kernel_launches"] - l0
+    return dict(first=first, psi=psi, last=snapshot(sf, cat.n_nodes, dts), launches=launches, wall=wall)
 
 
 def _switch_catchment(n_nodes):
@@ -158,10 +126,13 @@ def test_persistent_switch_point(product, checker, n_nodes, persistent):
     default = _with_mode(None, lambda: _first_steps_of_hour(product, cat))
     per_sweep = _with_mode("0", lambda: _first_steps_of_hour(product, cat))
     ref = _first_steps_of_hour(checker, cat)
-    _assert_matches_reference(cat, default, ref)
-    _assert_bit_identical(default["last"], per_sweep["last"], f"N={n_nodes}")
+    assert_lockstep(default["first"], ref["first"], ref["psi"])
+    compare(default["last"], ref["last"], exact=False, sweeps=True,
+            mbe_abs=1e-6 * np.sum(np.abs(cat.rain_sink_source(RAIN_MM_H))) * np.sum(ref["last"]["dts"]))
+    assert_bit_identical(default["last"], per_sweep["last"], f"N={n_nodes}, persistent vs per sweep")
     l1, l0 = default["launches"], per_sweep["launches"]
-    steps, approximations, sweeps = (int(v) for v in default["last"]["counters"])
+    steps = len(default["last"]["dts"])
+    approximations, sweeps = (int(v) for v in default["last"]["counters"])
     if persistent:      # at least (sweeps - solves) launches fewer (test_gpu_persistent_solve.test_launch_counts)
         assert l1 < l0 and l1 < l0 - (sweeps - approximations) + 1, \
             f"N={n_nodes}: the persistent solve did not run ({l1} launches, {l0} with one launch per sweep)"
@@ -179,7 +150,10 @@ def test_past_the_wide_cap(product, checker):
     assert cat.n_nodes == 1_903_616
     gpu = _first_steps_of_hour(product, cat)
     ref = _first_steps_of_hour(checker, cat)
-    _assert_matches_reference(cat, gpu, ref)
-    steps, approximations, sweeps = (int(v) for v in gpu["last"]["counters"])
+    assert_lockstep(gpu["first"], ref["first"], ref["psi"])
+    compare(gpu["last"], ref["last"], exact=False, sweeps=True,
+            mbe_abs=1e-6 * np.sum(np.abs(cat.rain_sink_source(RAIN_MM_H))) * np.sum(ref["last"]["dts"]))
+    steps = len(gpu["last"]["dts"])
+    approximations, sweeps = (int(v) for v in gpu["last"]["counters"])
     print(f"[wide cap] N={cat.n_nodes}: {steps} steps, {approximations} approximations, {sweeps} sweeps on both sides; "
           f"computeStep wall time: product {gpu['wall']:.2f} s, {checker.backend} {ref['wall']:.2f} s")

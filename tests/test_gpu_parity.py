@@ -1,17 +1,21 @@
 """Parity of the CUDA path (through the C ABI) with the oracle on identical inputs.
 
-Tolerances (fp64; the only arithmetic differences are CUDA libm vs glibc and reduction order):
-  lock-step single computeStep : |dH| <= 1e-9 * max(1, |psi|), |dtheta| <= 1e-10, same accepted dt,
+Tolerances (fp64; the only arithmetic differences are CUDA libm vs glibc and reduction order), applied by
+scenarios.assert_lockstep and scenarios.compare:
+  lock-step single computeStep : |dH| <= 1e-9 * max(1, |psi|), soil |dtheta| <= 1e-10, same accepted dt,
                                  same approximation count
-  trajectory (hours of storm)  : |dH| <= 1e-6 * max(1, |H|) (abs floor 1e-8 m), |dtheta| <= 1e-7,
-                                 boundary flow sums rel 1e-6, mass-balance error abs <= 1e-6 * sum|sink|
+  trajectory (hours of storm)  : same accepted-dt sequence and approximation count, |dH| <= 1e-6 * max(1, |H|),
+                                 |dtheta| <= 1e-7, |dSe| <= 1e-6, K rel 1e-6, link flow sums within 1e-6 of the
+                                 largest, boundary flow sums rel 1e-6 (+1e-12), total water rel 1e-9, the last
+                                 step's mass-balance error within 1e-6 of the rain volume (sum|sink| x duration)
   integer maps                 : bit-exact
 """
 import numpy as np
 import pytest
 
-from criteria3d_b200 import BoundaryType, Field
+from criteria3d_b200 import Field
 from criteria3d_b200.synth import Catchment, run_hours, setup
+from scenarios import assert_lockstep, compare, snapshot
 
 pytestmark = pytest.mark.gpu
 
@@ -44,39 +48,17 @@ def test_initial_state_and_storage(product, checker):
 def test_lockstep_single_step(product, checker):
     cat = Catchment(40, 32, 6)
     _both(product, checker, cat)
-    sink = np.zeros(cat.n_nodes)
-    sink[: cat.n_surface] = cat.rain_sink_source(20.0)
-    for sf in (product, checker):
-        assert sf.set_field(Field.WATER_SINK_SOURCE, 0, sink) == 0
-    dt_g, dt_o = product.computeStep(3600.0), checker.computeStep(3600.0)
-    assert dt_g == dt_o
-    cg, co = product.counters(), checker.counters()
-    assert cg["approximations"] == co["approximations"]
-    Hg, Ho = (s.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes) for s in (product, checker))
-    psi = checker.get_field(Field.MATRIC_POTENTIAL, 0, cat.n_nodes)
-    assert np.max(np.abs(Hg - Ho) / np.maximum(1.0, np.abs(psi))) <= 1e-9
-    Wg, Wo = (s.get_field(Field.WATER_CONTENT, 0, cat.n_nodes) for s in (product, checker))
-    assert np.max(np.abs(Wg - Wo)[cat.n_surface:]) <= 1e-10
+    a, b = (snapshot(sf, cat.n_nodes, run_hours(sf, cat, [20.0], max_steps=1)) for sf in (product, checker))
+    assert_lockstep(a, b, checker.get_field(Field.MATRIC_POTENTIAL, 0, cat.n_nodes))
 
 
 @pytest.mark.parametrize("shape,hours", [((40, 32, 6), [20.0, 40.0, 5.0]), ((64, 48, 10), [40.0, 25.0])])
 def test_trajectory(product, checker, shape, hours):
     cat = Catchment(*shape)
     _both(product, checker, cat)
-    dg, do = run_hours(product, cat, hours), run_hours(checker, cat, hours)
-    assert dg == do, "accepted time-step sequences differ"
-    Hg, Ho = (s.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes) for s in (product, checker))
-    assert np.max(np.abs(Hg - Ho) / np.maximum(1.0, np.abs(Ho))) <= 1e-6
-    Wg, Wo = (s.get_field(Field.WATER_CONTENT, 0, cat.n_nodes) for s in (product, checker))
-    assert np.max(np.abs(Wg - Wo)) <= 1e-7
-    for bt in (BoundaryType.Runoff, BoundaryType.FreeDrainage, BoundaryType.FreeLateralDrainage):
-        a, b = product.getTotalBoundaryWaterFlow(int(bt)), checker.getTotalBoundaryWaterFlow(int(bt))
-        assert a == pytest.approx(b, rel=1e-6, abs=1e-9), bt.name
-    assert product.getTotalWaterContent() == pytest.approx(checker.getTotalWaterContent(), rel=1e-9)
-    cg, co = product.counters(), checker.counters()
-    assert cg["steps"] == co["steps"] and cg["approximations"] == co["approximations"]
+    a, b = (snapshot(sf, cat.n_nodes, run_hours(sf, cat, hours)) for sf in (product, checker))
     sink_total = sum(np.sum(np.abs(cat.rain_sink_source(mm))) * 3600.0 for mm in hours)
-    assert abs(cg["last_mbe"] - co["last_mbe"]) <= 1e-6 * sink_total
+    compare(a, b, exact=False, mbe_abs=1e-6 * sink_total)
 
 
 def test_pattern_compressed_indices_are_bit_identical(product, checker, monkeypatch):

@@ -9,7 +9,7 @@ import pytest
 
 from criteria3d_b200 import Field
 from criteria3d_b200.synth import Catchment, run_hours, setup
-from scenarios import SCENARIOS, compare
+from scenarios import SCENARIOS, assert_bit_identical, compare
 
 pytestmark = pytest.mark.gpu
 
@@ -36,10 +36,7 @@ def test_both_solve_paths_match_the_reference_and_each_other(product, checker, n
     per = _with_mode("0", lambda: SCENARIOS[name](product))           # one launch per sweep
     compare(one, ref, exact=False)
     compare(per, ref, exact=False)
-    for key in one:
-        a, b = np.asarray(one[key]), np.asarray(per[key])
-        if a.dtype.kind in "fiu" and a.shape == b.shape:
-            assert np.array_equal(a, b, equal_nan=True), f"{name}: {key} differs between the two solve paths"
+    assert_bit_identical(one, per, f"{name}, persistent vs per sweep")
 
 
 def test_launch_counts(product):

@@ -10,8 +10,9 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from criteria3d_b200 import BoundaryType, Field, SoilFluxes3D
+from criteria3d_b200 import SoilFluxes3D
 from criteria3d_b200.synth import STORM_MM_H, Catchment, run_hours, setup
+from scenarios import compare, snapshot
 
 pytestmark = pytest.mark.gpu
 LIB = Path(__file__).resolve().parent.parent / "criteria3d_b200" / "libsf3d_b200_refround.so"
@@ -27,13 +28,9 @@ def test_reference_rounding_build_lockstep_over_two_storm_hours(checker):
     res = {}
     for name, lib in (("gpu", sf), ("ref", checker)):
         setup(lib, cat, threads=0)
-        dts = run_hours(lib, cat, mm)
-        res[name] = (dts, lib.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes), lib.get_field(Field.WATER_CONTENT, 0, cat.n_nodes),
-                     lib.getTotalBoundaryWaterFlow(int(BoundaryType.Runoff)), lib.counters())
-    (dg, Hg, Wg, rg, cg), (dr, Hr, Wr, rr, cr) = res["gpu"], res["ref"]
-    assert dg == dr, "accepted time-step sequence"
-    assert (cg["approximations"], cg["sweeps"]) == (cr["approximations"], cr["sweeps"])
-    assert np.max(np.abs(Hg - Hr)) <= 1e-7                     # metres, absolute, heads ~230 m (default build: 1e-6 relative = 2e-4 m); measured 2.4e-8
-    assert np.max(np.abs(Wg - Wr)) <= 1e-9
-    assert rg == pytest.approx(rr, rel=1e-9, abs=1e-12)
-    print(f"[refround] {len(dg)} steps, {cg['sweeps']} sweeps on both sides; max |dH| {np.max(np.abs(Hg - Hr)):.2e} m")
+        res[name] = snapshot(lib, cat.n_nodes, run_hours(lib, cat, mm))
+    g, r = res["gpu"], res["ref"]
+    # heads absolute in metres: ~230 m, so the default build's 1e-6 relative is 2e-4 m; measured 2.4e-8
+    compare(g, r, exact=False, sweeps=True, h_abs=1e-7, theta_abs=1e-9, totals_rel=1e-9)
+    print(f"[refround] {len(g['dts'])} steps, {int(g['counters'][1])} sweeps on both sides; "
+          f"max |dH| {np.max(np.abs(g['TOTAL_POTENTIAL'] - r['TOTAL_POTENTIAL'])):.2e} m")

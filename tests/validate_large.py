@@ -12,9 +12,10 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
-from criteria3d_b200 import BoundaryType, Field, SoilFluxes3D, load_product  # noqa: E402
+from criteria3d_b200 import SoilFluxes3D, load_product  # noqa: E402
 from oracle import ORACLE_LIB, REFERENCE_LIB  # noqa: E402
 from criteria3d_b200.synth import STORM_MM_H, Catchment, run_hours, setup  # noqa: E402
+from scenarios import snapshot  # noqa: E402
 
 
 def main():
@@ -24,26 +25,25 @@ def main():
     mm = STORM_MM_H[1:1 + hours]
     gpu = load_product()
     chk = SoilFluxes3D(REFERENCE_LIB if REFERENCE_LIB.exists() else ORACLE_LIB)
-    res = {}
+    res, wall = {}, {}
     for name, sf in (("gpu", gpu), ("oracle", chk)):
         setup(sf, cat, threads=0)
         t0 = time.perf_counter()
         dts = run_hours(sf, cat, mm)
-        res[name] = dict(dts=dts, wall=time.perf_counter() - t0, H=sf.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes),
-                         W=sf.get_field(Field.WATER_CONTENT, 0, cat.n_nodes), tw=sf.getTotalWaterContent(),
-                         bt=[sf.getTotalBoundaryWaterFlow(int(b)) for b in (BoundaryType.Runoff, BoundaryType.FreeDrainage,
-                                                                              BoundaryType.FreeLateralDrainage)],
-                         c=sf.counters())
+        wall[name] = time.perf_counter() - t0
+        res[name] = snapshot(sf, cat.n_nodes, dts)
     g, o = res["gpu"], res["oracle"]
-    same = g["dts"] == o["dts"]
-    first_div = next((k for k, (x, y) in enumerate(zip(g["dts"], o["dts"])) if x != y), None)
     out = {
         "grid": f"{rows}x{cols}x(1+{layers})", "nodes": cat.n_nodes, "hours_mm": mm, "checker": chk.backend,
-        "accepted_steps": [len(g["dts"]), len(o["dts"])], "dt_sequences_identical": same, "first_divergent_step": first_div,
-        "approximations": [g["c"]["approximations"], o["c"]["approximations"]], "sweeps": [g["c"]["sweeps"], o["c"]["sweeps"]],
-        "max_abs_dH": float(np.max(np.abs(g["H"] - o["H"]))), "max_abs_dtheta": float(np.max(np.abs(g["W"] - o["W"]))),
-        "total_water": [g["tw"], o["tw"]], "boundary_totals": [g["bt"], o["bt"]],
-        "mbe": [g["c"]["last_mbe"], o["c"]["last_mbe"]], "wall_s": [g["wall"], o["wall"]],
+        "accepted_steps": [len(g["dts"]), len(o["dts"])], "dt_sequences_identical": bool(np.array_equal(g["dts"], o["dts"])),
+        "first_divergent_step": next((k for k, (x, y) in enumerate(zip(g["dts"], o["dts"])) if x != y), None),
+        "approximations": [int(g["counters"][0]), int(o["counters"][0])], "sweeps": [int(g["counters"][1]), int(o["counters"][1])],
+        "max_abs_dH": float(np.max(np.abs(g["TOTAL_POTENTIAL"] - o["TOTAL_POTENTIAL"]))),
+        "max_abs_dtheta": float(np.max(np.abs(g["WATER_CONTENT"] - o["WATER_CONTENT"]))),
+        "total_water": [float(g["total_water"]), float(o["total_water"])],
+        # runoff, free and free lateral drainage, as in profiles/r01_parity_large.json
+        "boundary_totals": [g["boundary_totals"][:3].tolist(), o["boundary_totals"][:3].tolist()],
+        "mbe": [float(g["mbe_mbr"][0]), float(o["mbe_mbr"][0])], "wall_s": [wall["gpu"], wall["oracle"]],
     }
     Path(ROOT / "gpurun_out").mkdir(exist_ok=True)
     (ROOT / "gpurun_out" / "parity_large.json").write_text(json.dumps(out, indent=1))
