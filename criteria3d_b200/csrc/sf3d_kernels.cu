@@ -253,6 +253,9 @@ __device__ __forceinline__ double fold_partials(const double *part, double *sh)
 // ------------------------------------------------------------------------------------------
 // kernels
 // ------------------------------------------------------------------------------------------
+// a halo copy of a row that another rank owns (multi-GPU slabs)
+__device__ __forceinline__ bool sf3d_is_ghost(const SF3DView &v, uint32_t i) { return v.world > 1 && META_GHOST(v.meta[i]); }
+
 __global__ void __launch_bounds__(SF3D_BLOCK) kern_link_geometry(SF3DView v, int *orderOk)
 {
     const size_t N = v.N;
@@ -309,7 +312,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK) kern_build_patterns(SF3DView v, un
     const size_t N = v.N;
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
     {
-        if (v.world > 1 && META_GHOST(v.meta[i])) { pid[i] = SF3D_GHOST_PID; continue; }
+        if (sf3d_is_ghost(v, i)) { pid[i] = SF3D_GHOST_PID; continue; }
         int32_t off[SF3D_NLINK];
         bool fits = true;
         #pragma unroll
@@ -355,7 +358,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK) kern_verify_patterns(SF3DView v, c
     const size_t N = v.N;
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
     {
-        if (pid[i] == SF3D_GHOST_PID) { if (!(v.world > 1 && META_GHOST(v.meta[i]))) *mismatch = 1; continue; }
+        if (pid[i] == SF3D_GHOST_PID) { if (!sf3d_is_ghost(v, i)) *mismatch = 1; continue; }
         const int32_t *off = table + (size_t)pid[i] * SF3D_NLINK;
         #pragma unroll
         for (int c = 0; c < SF3D_NLINK; ++c)
@@ -532,6 +535,12 @@ struct HeatJacobiRule {
         else if (c->sweeps >= maxIter) c->status = SOLVE_MAXITER;
     }
 };
+template <bool HEAT>
+__host__ __device__ inline auto jacobi_rule(const SF3DView &v, int maxIter, double tol)
+{
+    if constexpr (HEAT) return HeatJacobiRule{maxIter, tol};
+    else return WaterJacobiRule{v.nGlobal, maxIter, tol};
+}
 struct WaterPostRule {
     static constexpr int count = 2; static constexpr bool isMax = false, whileRunning = false;
     __device__ void operator()(Ctrl *c, const double *r) const { c->storage = r[0]; c->sinkSum = r[1]; }
@@ -552,14 +561,16 @@ struct HeatCourantRule {
 // The end of every reducing kernel, after thread 0 stored the block's partial(s) in v.partA (and v.partB): the block
 // that finishes last folds the partials in a fixed order, then
 //   * one GPU: applies the rule;
-//   * peer transport (peer = true): all-reduces the values over the ranks through the mailboxes, applies the rule;
+//   * peer transport (several ranks, cm.mine set): all-reduces the values over the ranks through the mailboxes, applies
+//     the rule;
 //   * NCCL transport: leaves the local values in Ctrl::red (the host all-reduces them and launches kern_rule);
 // and resets the ticket.
 template <class Rule>
-__device__ __forceinline__ void finish_reduction(const SF3DView &v, double *sh, bool peer, const CommDev &cm, const Rule &rule)
+__device__ __forceinline__ void finish_reduction(const SF3DView &v, double *sh, const CommDev &cm, const Rule &rule)
 {
     Ctrl *c = v.ctrl;
     if (!last_block(c)) return;
+    const bool peer = v.world > 1 && cm.mine != nullptr;
     double r[2];
     r[0] = fold_partials<Rule::isMax>(v.partA, sh);
     if (Rule::count == 2) r[1] = fold_partials<Rule::isMax>(v.partB, sh);
@@ -608,13 +619,13 @@ __global__ void __launch_bounds__(SF3D_BLOCK, HEAT ? SF3D_HEAT_ASSEMBLE_BLOCKS :
     double courant = 0.;
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
     {
-        if (v.world > 1 && META_GHOST(v.meta[i])) continue;
+        if (sf3d_is_ghost(v, i)) continue;
         const double c = sf3d_row_assemble<HEAT>(v, i, dt, approx, ksh + threadIdx.x, SF3D_BLOCK);
         courant = (courant < c) ? c : courant;
     }
     courant = block_reduce<true>(courant, sh);
     if (threadIdx.x == 0) v.partA[blockIdx.x] = courant;
-    finish_reduction(v, sh, v.world > 1 && cm.mine != nullptr, cm, CourantRule{dt, dtMin});
+    finish_reduction(v, sh, cm, CourantRule{dt, dtMin});
 }
 
 // coupled heat: thermal liquid / vapour fluxes of every soil row (invariantFluxes of the water system), before the
@@ -625,7 +636,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK, HEAT ? SF3D_HEAT_ASSEMBLE_BLOCKS :
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_THERMAL_BLOCKS) kern_thermal_invariant(SF3DView v)
 {
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) sf3d_row_thermal_invariant(v, i);
+        if (!sf3d_is_ghost(v, i)) sf3d_row_thermal_invariant(v, i);
 }
 
 // one Jacobi sweep (Water::JacobiWaterCPU, sum of |dx|; heat: the infinity norm of heat.cpp:664-685) + the stopping
@@ -634,74 +645,66 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_THERMAL_BLOCKS) kern_thermal_
 #ifndef SF3D_JACOBI_BLOCKS
 #define SF3D_JACOBI_BLOCKS 8
 #endif
+// this thread's rows of one sweep (grid-stride), except those skip(i) is true for; the rows' norm terms are added to
+// norm (water) or raise it to their maximum (heat)
+template <bool HEAT, bool COHERENT = false, class Skip>
+__device__ __forceinline__ double sweep_rows(const SF3DView &v, const double *xin, double *xout, double norm, Skip skip)
+{
+    for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
+    {
+        if (skip(i)) continue;
+        const double d = HEAT ? sf3d_row_heat_jacobi(v, i, xin, xout) : sf3d_row_jacobi<COHERENT>(v, i, xin, xout);
+        norm = HEAT ? ((norm < d) ? d : norm) : (norm + d);
+    }
+    return norm;
+}
 template <bool HEAT>
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_JACOBI_BLOCKS) kern_jacobi(SF3DView v, const double *__restrict__ xin,
                                                           double *__restrict__ xout, int maxIter, double tol)
 {
     if (v.ctrl->status != SOLVE_RUNNING) return;
     __shared__ double sh[SF3D_BLOCK / 32];
-    double norm = 0.;
-    for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-    {
-        if (v.world > 1 && v.pid[i] == SF3D_GHOST_PID) continue;
-        const double d = HEAT ? sf3d_row_heat_jacobi(v, i, xin, xout) : sf3d_row_jacobi(v, i, xin, xout);
-        norm = HEAT ? ((norm < d) ? d : norm) : (norm + d);
-    }
+    double norm = sweep_rows<HEAT>(v, xin, xout, 0., [&](uint32_t i) { return v.world > 1 && v.pid[i] == SF3D_GHOST_PID; });
     norm = block_reduce<HEAT>(norm, sh);
     if (threadIdx.x == 0) v.partA[blockIdx.x] = norm;
-    if (HEAT) finish_reduction(v, sh, false, CommDev{}, HeatJacobiRule{maxIter, tol});
-    else finish_reduction(v, sh, false, CommDev{}, WaterJacobiRule{v.nGlobal, maxIter, tol});
+    finish_reduction(v, sh, CommDev{}, jacobi_rule<HEAT>(v, maxIter, tol));
 }
 
 // ---- small graphs: all sweeps of one solve in ONE launch -------------------------------------------------
 // A catchment of a few ten thousand nodes (BASELINE config 1, CRITERIA-1D-sized callers) sweeps in ~1 us, so a solve of
 // 30 sweeps is bound by 30 launches and by the batches' control-block reads.  This kernel is launched cooperatively
 // (every block resident) and iterates on the device: sweep, block partial, grid-wide barrier, EVERY block folds the
-// partials in the same fixed order and applies the stopping rule of cpusolver.cpp:678-700 to its own copy of the
-// solver state, so all blocks leave the loop in the same sweep without a second barrier; the partials alternate
-// between two arrays, so a fast block's next partial never lands in the array a slow block is still folding.  Grid
-// size, thread -> row mapping, partial sums and fold order are those of kern_jacobi: the residual norms, and with them
-// the decisions, are bit-identical to the launch-per-sweep path.  xa holds the solution at entry.
+// partials in the same fixed order and applies the stopping rule of kern_jacobi to its own copy of the solver state,
+// so all blocks leave the loop in the same sweep without a second barrier; the partials alternate between two
+// arrays, so a fast block's next partial never lands in the array a slow block is still folding.  Grid size, thread
+// -> row mapping, partial sums and fold order are those of kern_jacobi: the residual norms, and with them the
+// decisions, are bit-identical to the launch-per-sweep path.  xa holds the solution at entry.
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_JACOBI_BLOCKS) kern_jacobi_persistent(SF3DView v, double *xa, double *xb, int maxIter, double tol)
 {
     cooperative_groups::grid_group grid = cooperative_groups::this_grid();
-    Ctrl *c = v.ctrl;
-    if (c->status != SOLVE_RUNNING) return;             // Courant failure of the assembly: the same branch in every block
+    if (v.ctrl->status != SOLVE_RUNNING) return;        // Courant failure of the assembly: the same branch in every block
     __shared__ double sh[SF3D_BLOCK / 32];
-    __shared__ int shStatus;
-    double best = c->bestNorm, curr = 0.;               // thread 0's copy of the solver state (identical in every block)
-    int sweeps = 0, status = SOLVE_RUNNING;
-    for (;;)
+    __shared__ int status;
+    // thread 0's copy of the solver state (identical in every block), in registers: the rule is on the critical path of
+    // every sweep
+    Ctrl c = *v.ctrl;
+    const auto rule = jacobi_rule<false>(v, maxIter, tol);
+    for (int sweep = 0; ; ++sweep)
     {
-        const double *xin = (sweeps & 1) ? xb : xa;
-        double *xout = (sweeps & 1) ? xa : xb;
-        double *part = (sweeps & 1) ? v.partB : v.partA;
-        double norm = 0.;
-        for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-            norm += sf3d_row_jacobi_coherent(v, i, xin, xout);
+        const double *xin = (sweep & 1) ? xb : xa;
+        double *xout = (sweep & 1) ? xa : xb;
+        double *part = (sweep & 1) ? v.partB : v.partA;
+        double norm = sweep_rows<false, true>(v, xin, xout, 0., [](uint32_t) { return false; });
         norm = block_reduce<false>(norm, sh);
         if (threadIdx.x == 0) part[blockIdx.x] = norm;
         grid.sync();
         const double total = fold_partials<false>(part, sh);
-        ++sweeps;
-        if (threadIdx.x == 0)
-        {
-            curr = total / v.nGlobal;                                       // water.cpp:600
-            int st = SOLVE_RUNNING;
-            if (curr < tol) st = SOLVE_CONVERGED;                           // cpusolver.cpp:692
-            else if (curr > best * 10) st = SOLVE_DIVERGED;                 // :695
-            else
-            {
-                if (curr < best) best = curr;                               // :698
-                if (sweeps >= maxIter) st = SOLVE_MAXITER;
-            }
-            shStatus = st;
-        }
+        if (threadIdx.x == 0) { rule(&c, &total); status = c.status; }
         __syncthreads();
-        status = shStatus;
         if (status != SOLVE_RUNNING) break;
     }
-    if (blockIdx.x == 0 && threadIdx.x == 0) { c->lastNorm = curr; c->sweeps = sweeps; c->bestNorm = best; c->status = status; }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+    { v.ctrl->lastNorm = c.lastNorm; v.ctrl->sweeps = c.sweeps; v.ctrl->bestNorm = c.bestNorm; v.ctrl->status = c.status; }
 }
 
 // NCCL transport: gather owned boundary values into the send buffer / scatter received ones into the ghost rows
@@ -763,16 +766,11 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_JACOBI_BLOCKS) kern_jacobi_mu
         // block's own fence, before the sequence number the peers wait for
         __threadfence_system();
     }
-    for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-    {
-        if ((v.pid[i] & SF3D_PID_SKIP) != 0) continue;         // ghost row, or boundary row already done above
-        const double d = HEAT ? sf3d_row_heat_jacobi(v, i, xin, xout) : sf3d_row_jacobi(v, i, xin, xout);
-        norm = HEAT ? ((norm < d) ? d : norm) : (norm + d);
-    }
+    // ghost rows, and the boundary rows done above, are skipped
+    norm = sweep_rows<HEAT>(v, xin, xout, norm, [&](uint32_t i) { return (v.pid[i] & SF3D_PID_SKIP) != 0; });
     norm = block_reduce<HEAT>(norm, sh);
     if (threadIdx.x == 0) v.partA[blockIdx.x] = norm;
-    if (HEAT) finish_reduction(v, sh, true, cm, HeatJacobiRule{maxIter, tol});
-    else finish_reduction(v, sh, true, cm, WaterJacobiRule{v.nGlobal, maxIter, tol});
+    finish_reduction(v, sh, cm, jacobi_rule<HEAT>(v, maxIter, tol));
 }
 __global__ void __launch_bounds__(SF3D_BLOCK) kern_mark_boundary(uint16_t *pid, const uint32_t *__restrict__ idx, uint32_t n)
 {
@@ -804,14 +802,14 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_POST_BLOCKS) kern_post(SF3DVi
     {
         double s, q;
         sf3d_row_post(v, i, x, dt, mode, &s, &q);
-        if (v.world > 1 && META_GHOST(v.meta[i])) continue;      // ghosts are counted by their owner
+        if (sf3d_is_ghost(v, i)) continue;      // ghosts are counted by their owner
         storage += s;
         sinkSum += q;
     }
     storage = block_reduce<false>(storage, sh);
     sinkSum = block_reduce<false>(sinkSum, sh);
     if (threadIdx.x == 0) { v.partA[blockIdx.x] = storage; v.partB[blockIdx.x] = sinkSum; }
-    finish_reduction(v, sh, v.world > 1 && cm.mine != nullptr, cm, WaterPostRule{});
+    finish_reduction(v, sh, cm, WaterPostRule{});
 }
 
 // PREP: the copies of the next try's first pass (kern_begin_try) ride on this pass (water-only runs: the heat step
@@ -821,7 +819,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK) kern_accept(SF3DView v, double dt)
 {
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
     {
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) sf3d_row_accept(v, i, dt);
+        if (!sf3d_is_ghost(v, i)) sf3d_row_accept(v, i, dt);
         if (PREP) sf3d_row_prepare_try(v, i);
     }
 }
@@ -838,10 +836,10 @@ __global__ void __launch_bounds__(SF3D_BLOCK) kern_total_boundary(SF3DView v, ui
     __shared__ double sh[SF3D_BLOCK / 32];
     double sum = 0.;
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-        if (META_BT(v.meta[i]) == bt && !(v.world > 1 && META_GHOST(v.meta[i]))) sum += v.bSum[i];
+        if (META_BT(v.meta[i]) == bt && !sf3d_is_ghost(v, i)) sum += v.bSum[i];
     sum = block_reduce<false>(sum, sh);
     if (threadIdx.x == 0) v.partA[blockIdx.x] = sum;
-    finish_reduction(v, sh, v.world > 1 && cm.mine != nullptr, cm, BoundaryTotalRule{});
+    finish_reduction(v, sh, cm, BoundaryTotalRule{});
 }
 
 // setNodeMatricPotential / setNodeTotalPotential over a range (soilFluxes3D.cpp:869-906)
@@ -1013,7 +1011,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_coeffs
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_save_water_fluxes(SF3DView v, double dtHeat, double dtWater)
 {
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) sf3d_row_save_water_fluxes(v, i, dtHeat, dtWater);    // a ghost row has no link pattern
+        if (!sf3d_is_ghost(v, i)) sf3d_row_save_water_fluxes(v, i, dtHeat, dtWater);    // a ghost row has no link pattern
 }
 // updateBoundaryHeatData: heat flux per node + max heat-boundary Courant (heat.cpp:237-340)
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_boundary_heat(SF3DView v, double maxTimeStep, CommDev cm)
@@ -1023,11 +1021,11 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_boundary_he
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
     {
         const double c = sf3d_row_boundary_heat(v, i, maxTimeStep);
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) courant = (courant < c) ? c : courant;
+        if (!sf3d_is_ghost(v, i)) courant = (courant < c) ? c : courant;
     }
     courant = block_reduce<true>(courant, sh);
     if (threadIdx.x == 0) v.partA[blockIdx.x] = courant;
-    finish_reduction(v, sh, v.world > 1 && cm.mine != nullptr, cm, HeatCourantRule{});
+    finish_reduction(v, sh, cm, HeatCourantRule{});
 }
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_begin(SF3DView v, double dtHeat, double dtWater)
 {
@@ -1046,7 +1044,7 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_begin(
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_assemble(SF3DView v, double dtHeat, double dtWater)
 {
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) sf3d_row_heat_assemble(v, i, dtHeat, dtWater);
+        if (!sf3d_is_ghost(v, i)) sf3d_row_heat_assemble(v, i, dtHeat, dtWater);
 }
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_post(SF3DView v, const double *__restrict__ x, double dtHeat,
                                                              double dtWater, int mode, CommDev cm)
@@ -1057,18 +1055,18 @@ __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_post(S
     {
         double s, q;
         sf3d_row_heat_post(v, i, x, dtHeat, dtWater, mode, &s, &q);
-        if (v.world > 1 && META_GHOST(v.meta[i])) continue;
+        if (sf3d_is_ghost(v, i)) continue;
         storage += s; sinkSum += q;
     }
     storage = block_reduce<false>(storage, sh);
     sinkSum = block_reduce<false>(sinkSum, sh);
     if (threadIdx.x == 0) { v.partA[blockIdx.x] = storage; v.partB[blockIdx.x] = sinkSum; }
-    finish_reduction(v, sh, v.world > 1 && cm.mine != nullptr, cm, HeatPostRule{});
+    finish_reduction(v, sh, cm, HeatPostRule{});
 }
 __global__ void __launch_bounds__(SF3D_BLOCK, SF3D_HEAT_BLOCKS) kern_heat_accept(SF3DView v, double dtHeat, double dtWater)
 {
     for (uint32_t i = blockIdx.x * SF3D_BLOCK + threadIdx.x; i < v.N; i += gridDim.x * SF3D_BLOCK)
-        if (!(v.world > 1 && META_GHOST(v.meta[i]))) sf3d_row_heat_accept(v, i, dtHeat, dtWater);
+        if (!sf3d_is_ghost(v, i)) sf3d_row_heat_accept(v, i, dtHeat, dtWater);
 }
 // mode 0: oldT = T (accepted, cpusolver.cpp:598-602); mode 1: T = oldT (refused, :582-588)
 __global__ void __launch_bounds__(SF3D_BLOCK) kern_heat_copy_T(SF3DView v, int mode)
@@ -1504,8 +1502,8 @@ void k_jacobi_persistent(const SF3DView &v, double *xa, double *xb, int maxIter,
 }
 // one sweep.  Peer transport: one launch (boundary rows first with peer stores, interior rows, in-kernel all-reduce +
 // stopping rule).  One GPU: one launch.  NCCL: the sweep, the halo exchange, the all-reduce of the norm and the rule.
-template <bool HEAT, class Rule>
-static void jacobi_sweep(const SF3DView &v, const double *xin, double *xout, int maxIter, double tol, int kind, const Rule &rule)
+template <bool HEAT>
+static void jacobi_sweep(const SF3DView &v, const double *xin, double *xout, int maxIter, double tol, int kind)
 {
     const Transport t = transport(v);
     {
@@ -1514,10 +1512,10 @@ static void jacobi_sweep(const SF3DView &v, const double *xin, double *xout, int
         else kern_jacobi<HEAT><<<GRID(v.N)>>>(v, xin, xout, maxIter, tol);
         LAUNCH_CHECK();
     }
-    if (t == TRANSPORT_NCCL) { ProfScope ps(SF3D_K_COMM); nccl_halo(xout); nccl_finish(v, rule); }
+    if (t == TRANSPORT_NCCL) { ProfScope ps(SF3D_K_COMM); nccl_halo(xout); nccl_finish(v, jacobi_rule<HEAT>(v, maxIter, tol)); }
 }
 void k_jacobi(const SF3DView &v, const double *xin, double *xout, int maxIter, double tol)
-{ jacobi_sweep<false>(v, xin, xout, maxIter, tol, SF3D_K_JACOBI, WaterJacobiRule{v.nGlobal, maxIter, tol}); }
+{ jacobi_sweep<false>(v, xin, xout, maxIter, tol, SF3D_K_JACOBI); }
 void k_post(const SF3DView &v, const double *x, double dt, int mode)
 {
     { ProfScope ps(SF3D_K_POST); kern_post<<<GRID(v.N)>>>(v, x, dt, mode, comm_dev(v)); LAUNCH_CHECK(); }
@@ -1591,7 +1589,7 @@ void k_heat_begin(const SF3DView &v, double dtHeat, double dtWater, bool coeffsA
 void k_heat_assemble(const SF3DView &v, double dtHeat, double dtWater)
 { ProfScope ps(SF3D_K_HEAT_ASSEMBLE); kern_heat_assemble<<<GRID(v.N)>>>(v, dtHeat, dtWater); LAUNCH_CHECK(); }
 void k_heat_jacobi(const SF3DView &v, const double *xin, double *xout, int maxIter, double tol)
-{ jacobi_sweep<true>(v, xin, xout, maxIter, tol, SF3D_K_HEAT_JACOBI, HeatJacobiRule{maxIter, tol}); }
+{ jacobi_sweep<true>(v, xin, xout, maxIter, tol, SF3D_K_HEAT_JACOBI); }
 void k_heat_post(const SF3DView &v, const double *x, double dtHeat, double dtWater, int mode)
 {
     ProfScope ps(SF3D_K_HEAT_POST);

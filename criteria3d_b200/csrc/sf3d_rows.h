@@ -536,7 +536,16 @@ SF3D_HD double sf3d_row_assemble(const SF3DView &v, uint32_t i, double dt, int a
 
 // ==========================================================================================
 // Water::JacobiWaterCPU, one row (water.cpp:570-596).  Returns the row's contribution to the norm.
+// COHERENT: the row of the persistent small-graph solve (all sweeps of a solve in ONE kernel, grid-wide barrier
+// between sweeps): the solution vectors are written by other thread blocks earlier in the same launch, so they are
+// read through L2 (ld.global.cg) and never through the non-coherent read-only path.  Same operations in the same order.
 // ==========================================================================================
+#if defined(__CUDA_ARCH__)
+#define SF3D_LDCG(p) __ldcg(p)
+#else
+#define SF3D_LDCG(p) (*(p))
+#endif
+template <bool COHERENT = false>
 SF3D_HD double sf3d_row_jacobi(const SF3DView &v, uint32_t i, const double *__restrict__ xin, double *__restrict__ xout,
                                double *xnewOut = nullptr)
 {
@@ -548,46 +557,16 @@ SF3D_HD double sf3d_row_jacobi(const SF3DView &v, uint32_t i, const double *__re
     for (int c = 0; c < SF3D_NLINK; ++c)
     {
         const double A = SF3D_LDS(v.mval + (size_t)c * N + i);
-        xnew -= A * xin[j[c]];
+        xnew -= A * (COHERENT ? SF3D_LDCG(xin + j[c]) : xin[j[c]]);
     }
     const double z = SF3D_LDS(v.z + i);
     if (i < v.Ns) xnew = sf3d_max(xnew, z);
-    const double xold = xin[i];
+    const double xold = COHERENT ? SF3D_LDCG(xin + i) : xin[i];
     double norm = fabs(xnew - xold);
     const double psi = fabs(xnew - z);
     if (psi > 1.) norm *= (1. / psi);
     xout[i] = xnew;
     if (xnewOut) *xnewOut = xnew;
-    return norm;
-}
-
-// The same row for the persistent small-graph solve (all sweeps of a solve in ONE kernel, grid-wide barrier between
-// sweeps): the solution vectors are written by other thread blocks earlier in the same launch, so they are read
-// through L2 (ld.global.cg) and never through the non-coherent read-only path.  Same operations in the same order.
-#if defined(__CUDA_ARCH__)
-#define SF3D_LDCG(p) __ldcg(p)
-#else
-#define SF3D_LDCG(p) (*(p))
-#endif
-SF3D_HD double sf3d_row_jacobi_coherent(const SF3DView &v, uint32_t i, const double *xin, double *xout)
-{
-    const size_t N = v.N;
-    uint32_t j[SF3D_NLINK];
-    sf3d_row_cols(v, i, j);
-    double xnew = SF3D_LDS(v.b + i);
-    #pragma unroll
-    for (int c = 0; c < SF3D_NLINK; ++c)
-    {
-        const double A = SF3D_LDS(v.mval + (size_t)c * N + i);
-        xnew -= A * SF3D_LDCG(xin + j[c]);
-    }
-    const double z = SF3D_LDS(v.z + i);
-    if (i < v.Ns) xnew = sf3d_max(xnew, z);
-    const double xold = SF3D_LDCG(xin + i);
-    double norm = fabs(xnew - xold);
-    const double psi = fabs(xnew - z);
-    if (psi > 1.) norm *= (1. / psi);
-    xout[i] = xnew;
     return norm;
 }
 

@@ -820,8 +820,8 @@ SF3D_HD void sf3d_row_heat_assemble(const SF3DView &v, uint32_t i, double dtHeat
 // one Jacobi row of the heat system; returns |dx| (the reference sweeps Gauss-Seidel in place with
 // the same row formula and an infinity norm, heat.cpp:664-685; see DESIGN.md, Q6).  Entries are stored and
 // summed in SLOT order (= the reference's column order Up, Down, Lateral 0..7); the linked node of a slot comes
-// from the row's link pattern like in the water sweep (absent links and links to surface nodes hold a zero
-// entry pointing at the row itself / at a finite x), so no index array and no meta word are read.
+// from sf3d_row_cols like in the water sweep (absent links and links to surface nodes hold a zero entry pointing at
+// the row itself / at a finite x), so no meta word is read.
 SF3D_HD double sf3d_row_heat_jacobi(const SF3DView &v, uint32_t i, const double *__restrict__ xin, double *__restrict__ xout,
                                     double *xnewOut = nullptr)
 {
@@ -830,17 +830,7 @@ SF3D_HD double sf3d_row_heat_jacobi(const SF3DView &v, uint32_t i, const double 
     if (xnewOut) *xnewOut = xold;
     if (i < v.Ns || SF3D_LDS(v.hdiag + i) == 0.) { xout[i] = xold; return 0.; }
     uint32_t j[SF3D_NLINK];
-    if (v.pattern) sf3d_row_cols(v, i, j);      // j[c]: COLUMN order (Up, Lateral 0..7, Down)
-    else
-    {
-        const uint32_t m = v.meta[i];
-        #pragma unroll
-        for (int c = 0; c < SF3D_NLINK; ++c)
-        {
-            const int slot = sf3d_slot_of_col(c);
-            j[c] = META_HAS_SLOT(m, slot) ? v.lidx[(size_t)slot * N + i] : i;
-        }
-    }
+    sf3d_row_cols(v, i, j);                     // j[c]: COLUMN order (Up, Lateral 0..7, Down)
     double xnew = SF3D_LDS(v.b + i);
     #pragma unroll
     for (int slot = 0; slot < SF3D_NLINK; ++slot)

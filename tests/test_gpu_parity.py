@@ -15,7 +15,7 @@ import pytest
 
 from criteria3d_b200 import Field
 from criteria3d_b200.synth import Catchment, run_hours, setup
-from scenarios import assert_lockstep, compare, snapshot
+from scenarios import assert_bit_identical, assert_lockstep, compare, heat_coupled, snapshot
 
 pytestmark = pytest.mark.gpu
 
@@ -61,19 +61,22 @@ def test_trajectory(product, checker, shape, hours):
     compare(a, b, exact=False, mbe_abs=1e-6 * sink_total)
 
 
-def test_pattern_compressed_indices_are_bit_identical(product, checker, monkeypatch):
-    """The sweep reads the column indices through 16-bit link patterns (2 B/node instead of 40 B).
-    The map is verified on the device at finalize; forcing the explicit index array must give
-    bit-identical potentials (integer work: exact)."""
+def _storm_25_steps(sf):
     cat = Catchment(33, 27, 5)
-    runs = []
-    for explicit in (False, True):
-        if explicit:
-            monkeypatch.setenv("SF3D_EXPLICIT_INDEX", "1")
-        else:
-            monkeypatch.delenv("SF3D_EXPLICIT_INDEX", raising=False)
-        setup(product, cat)
-        dts = run_hours(product, cat, [30.0], max_steps=25)
-        runs.append((dts, product.get_field(Field.TOTAL_POTENTIAL, 0, cat.n_nodes), product.counters()["sweeps"]))
-    assert runs[0][0] == runs[1][0] and runs[0][2] == runs[1][2]
-    assert np.array_equal(runs[0][1], runs[1][1])
+    setup(sf, cat)
+    return snapshot(sf, cat.n_nodes, run_hours(sf, cat, [30.0], max_steps=25))
+
+
+def test_pattern_compressed_indices_are_bit_identical(product, checker, monkeypatch):
+    """The sweeps read the column indices through 16-bit link patterns (2 B/node instead of 40 B).
+    The map is verified on the device at finalize; forcing the explicit index array must give
+    bit-identical results (integer work: exact), for the water sweep and for the heat sweep."""
+    for name, scenario in (("water", _storm_25_steps), ("heat", heat_coupled)):
+        runs = []
+        for explicit in (False, True):
+            if explicit:
+                monkeypatch.setenv("SF3D_EXPLICIT_INDEX", "1")
+            else:
+                monkeypatch.delenv("SF3D_EXPLICIT_INDEX", raising=False)
+            runs.append(scenario(product))
+        assert_bit_identical(runs[0], runs[1], f"{name}: explicit vs pattern-compressed indices")
